@@ -352,8 +352,7 @@ def run_loop(args):
         dist.init_process_group("nccl", device_id=dev)
     L = capi.lib()
     K, Wm, pre = args.steps, args.warmup, args.preroll
-    Kp = max(K, 100)                               # the profiled pass (roofline of the stencil, stage times) always covers >= 100 launches, whatever --steps
-    total = pre + Wm + 2 * K + Kp                  # pre-roll, warm-up, timed pass, profiled pass, end-to-end pass: one continuous stream
+    total = pre + Wm + 3 * K                       # pre-roll, warm-up, timed pass, profiled pass, end-to-end pass: one continuous stream
     P = default_params(W, H)
     P.maxNumFrames = total + 8
     P.maxNumImages = total // 10 + 8
@@ -374,10 +373,11 @@ def run_loop(args):
         d, c, _ = synth_gpu.make_frames(idx, W, H, device=str(dev), texture="rich")
         depth[s0:s0 + len(idx)] = d; color[s0:s0 + len(idx)] = c
     torch.cuda.synchronize()
-    f_e2e0 = pre + Wm + K + Kp
+    f_e2e0 = pre + Wm + 2 * K
     ahead = os.environ.get("BF_LOOP_AHEAD", "1") != "0"      # bfFrameLoopStepAhead: frame k + 1 of a pass is announced while frame k is stepped
     h_depth = depth[f_e2e0:f_e2e0 + K].cpu().pin_memory(); h_color = color[f_e2e0:f_e2e0 + K].cpu().pin_memory()
     stats = {"valid": 0, "local": 0, "local_valid": 0, "global": 0, "reint": 0, "kp": 0, "n": 0}
+    last = {}                                              # status block of the most recent step
 
     trace = []
 
@@ -411,6 +411,7 @@ def run_loop(args):
                 st = loop.step(h_depth[k], h_color[k], *((h_depth[k + 1], h_color[k + 1]) if la else (None, None)))
             else:
                 st = loop.step(depth[f0 + k], color[f0 + k], *((depth[f0 + k + 1], color[f0 + k + 1]) if la else (None, None)))
+            last["st"] = st
             if not profile:
                 note(st)
             if steptimes is not None:
@@ -435,10 +436,12 @@ def run_loop(args):
     if args.cuda_profiler:
         torch.cuda.profiler.stop()
     clk_mark1 = len(clk_lines)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, L, loop, last["st"], pre + Wm + K)
     c_before = loop.counters()
     prev_lanes = L.bfTsdfSetLanes(0)                       # the stencil is timed alone on its stream: the burst HBM peak is its roof
     loop.set_profiling(True)
-    timed(pre + Wm + K, Kp, False, True)
+    timed(pre + Wm + K, K, False, True)
     stages = loop.stage_times()
     loop.set_profiling(False)
     L.bfTsdfSetLanes(prev_lanes)
@@ -498,7 +501,7 @@ def run_loop(args):
         "streams": ("three" if ahead and overlap else "two" if ahead or overlap else "one") + " (bundling on the library stream" + ("; reconstruction on the loop's second stream" if overlap else "") +
                    ("; the NEXT frame's upload / ingest / SIFT detection / dense cache on the loop's feature stream (bfFrameLoopStepAhead, frames announced inside a pass only)" if ahead else "") +
                    "; events keep the single-threaded order's dependencies, results identical: tests/test_frame_loop_gpu.py)",
-        "stages_ms_per_step": dict(stages, note="profiled pass (>= 100 steps, serial on one stream, one extra host synchronisation per step, TSDF lanes off): device time line between stage boundaries, mean per step"),
+        "stages_ms_per_step": dict(stages, note="profiled pass (--steps steps, serial on one stream, one extra host synchronisation per step, TSDF lanes off): device time line between stage boundaries, mean per step"),
         "clocks": summarize_clocks(clk_lines[clk_mark0:clk_mark1]), "clocks_profile_pass": summarize_clocks(clk_lines[clk_mark1:clk_mark2]),
     }
     if world == 1 and os.environ.get("BF_BENCH_MESH", "1") != "0":
@@ -636,6 +639,42 @@ def run_sweep(args):
         dist.destroy_process_group()
 
 # ------------------------------------------------------------------------------------------------------------------------
+DUMP_BLOCKS = 2048               # voxel blocks of the fused model written by --dump-outputs (2048 x 512 voxels x 24 B = 25 MB)
+
+
+def dump_outputs(out_dir, L, loop, st, n_frames):
+    """--dump-outputs: what the timed pass computed in its last step, as a caller of bfFrameLoopStep receives it -- the status block (the frame's
+    pose and counters), the trajectory of every frame so far, and the fused model: the voxel words (sdf, weight, colour) of a fixed sample of its
+    blocks, in the order of their block coordinates (which hash slot a block occupies depends on scheduling; the block set and its voxels do not).
+    A block is sampled by a hash of its own coordinates, so two runs whose block sets differ by a few blocks still sample the same blocks elsewhere."""
+    from bundlefusion_b200 import _capi as capi
+    os.makedirs(out_dir, exist_ok=True)
+    save = lambda name, a: np.save(os.path.join(out_dir, name + ".npy"), a)
+    loop.join()
+    d = st.as_dict()
+    save("pose", d.pop("transform"))
+    for k, v in d.items():
+        save("status_" + k, np.array([v], np.float64))
+    save("trajectory", loop.trajectory(n_frames))
+    rt = ctypes.CDLL("libcudart.so.12")                    # the runtime the library is linked against (loaded with it)
+    rt.cudaMemcpy.argtypes = [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_size_t, ctypes.c_int]
+    hd, hp = L.bfFrameLoopGetHashData(loop._h).contents, L.bfFrameLoopGetHashParams(loop._h).contents
+    ent = np.empty((int(hp.m_hashNumBuckets) * capi.BF_HASH_BUCKET_SIZE, 8), np.int32)
+    capi.check(rt.cudaMemcpy(ent.ctypes.data, hd.d_hash, ent.nbytes, 2), "cudaMemcpy")
+    ent = ent[ent[:, 3] != -2]                                                          # allocated entries: (x, y, z, voxel offset, ...)
+    ent = ent[np.lexsort((ent[:, 2], ent[:, 1], ent[:, 0]))]
+    x, y, z = (ent[:, k].astype(np.int64) for k in range(3))
+    h = ((x * 73856093) ^ (y * 19349669) ^ (z * 83492791)) & 0xFFFFFFFF
+    pick = np.sort(np.argsort(h, kind="stable")[:DUMP_BLOCKS])
+    vox = np.empty((len(pick), capi.BF_SDF_BLOCK_VOXELS, 3), np.int32)
+    for i, e in enumerate(ent[pick]):
+        capi.check(rt.cudaMemcpy(vox[i].ctypes.data, hd.d_SDFBlocks + int(e[3]) * 12, vox[i].nbytes, 2), "cudaMemcpy")
+    save("tsdf_block_coords", ent[pick, :3].astype(np.float64))
+    save("tsdf_sdf", np.ascontiguousarray(vox[..., 0]).view(np.float32))
+    save("tsdf_weight", np.ascontiguousarray(vox[..., 1]).view(np.float32))
+    save("tsdf_color", np.ascontiguousarray(vox[..., 2]).view(np.uint8).reshape(len(pick), -1, 4).astype(np.float32))
+
+
 def mesh_leg(L, loop, P, dev, active_blocks):
     """Row N4: the iso-surface of the model the loop just built (bfMarchingCubesExtract on the loop's hash), timed with CUDA events on the library's stream -- the
     kernel's first hardware timing comes from this leg.  Runs after every other measurement of the line; a failure is reported in the entry, not raised."""
@@ -886,7 +925,10 @@ def main():
     ap.add_argument("--preroll", type=int, default=250, help="frames streamed through the loop before warm-up (state of a long stream)")
     ap.add_argument("--trace", default=None, help="diagnostic: write the per-frame status of every step (pre-roll included) to this file")
     ap.add_argument("--stride", type=int, default=2, help="Lissajous path frames per step")
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR", help="write what the timed pass computed in its last step to DIR/<name>.npy (frame-loop workload)")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl != "ours" or args.workload != "loop"):
+        ap.error("--dump-outputs writes the outputs of the frame-loop workload (--impl ours --workload loop)")
     if args.warmup < 3 and args.impl == "ours":
         args.warmup = 3
     if args.impl == "reference":

@@ -13,6 +13,7 @@ import numpy as np
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
 from bundlefusion_b200 import _capi as capi                                                                                   # noqa: E402
+from tests._golden import as_crc                                                                                                 # noqa: E402
 from tests.test_manager_reference_emulated import INGEST, area_problems, dense_problem, filter_problems, image_cases, trajectory_case    # noqa: E402
 
 F = np.float32
@@ -92,7 +93,7 @@ def main():
             wi, hi = int(W * fw), int(H * fh)
             raw, filt, od, oc = depth.copy(), np.zeros((H, W), F), np.zeros((hi, wi), F), np.zeros((hi, wi, 4), np.uint8)
             R.refIngestFrame(raw.ctypes.data, filt.ctypes.data, W, H, color.ctypes.data, W, H, wi, hi, erode, 3, 0.05, 0.3, sig, 0.05, od.ctypes.data, oc.ctypes.data)
-            out[f"ingest{k}_{c}_depth"], out[f"ingest{k}_{c}_color"] = od, oc
+            out.update(as_crc(f"ingest{k}_{c}_depth", od)); out.update(as_crc(f"ingest{k}_{c}_color", oc))      # shape + CRC32: whole frames would pass 1 MB
         print("images", k, W, H)
     tc = trajectory_case()
     n = len(tc["inval"])

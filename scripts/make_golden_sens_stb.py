@@ -11,6 +11,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
+from tests._golden import as_crc                                                 # noqa: E402
 from tests.test_sens_reference_stb import GOLDEN, RefStb, make_streams              # noqa: E402
 
 
@@ -20,14 +21,14 @@ def main():
     out = {"num_jpeg": np.int32(len(jpegs)), "num_png": np.int32(len(pngs)), "depth": depth}
     for i, b in enumerate(jpegs):
         out[f"jpeg_{i}"] = np.frombuffer(b, np.uint8)
-        out[f"jpeg_rgb_{i}"] = R.decode(b)
+        out.update(as_crc(f"jpeg_rgb_{i}", R.decode(b)))                            # shape + CRC32: the decoded pixels whole would pass 1 MB
     for i, b in enumerate(pngs):
         out[f"png_{i}"] = np.frombuffer(b, np.uint8)
         out[f"png_rgb_{i}"] = R.decode(b)
     z = R.zlib_compress(depth.tobytes(), 8)                                          # RGBDFrame::compressDepth's quality
     assert R.zlib_decode(z, depth.nbytes) == depth.tobytes()
     out["depth_stb_zlib"] = np.frombuffer(z, np.uint8)
-    out["sens_jpeg_ids"] = np.array([i for i, b in enumerate(jpegs) if out[f"jpeg_rgb_{i}"].shape == (120, 160, 3)], np.int32)
+    out["sens_jpeg_ids"] = np.array([i for i, b in enumerate(jpegs) if tuple(out[f"jpeg_rgb_{i}_shape"]) == (120, 160, 3)], np.int32)
     np.savez_compressed(GOLDEN, **out)
     print("wrote", GOLDEN, os.path.getsize(GOLDEN), "bytes;", len(jpegs), "jpeg,", len(pngs), "png streams")
 

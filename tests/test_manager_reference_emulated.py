@@ -11,6 +11,7 @@ import numpy as np
 
 from bundlefusion_b200 import synth
 from oracle import oracle as orc
+from tests._golden import matches
 from tests.test_verify_filters_oracle import VERIFY
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -186,7 +187,7 @@ def test_cache_frame_and_ingest():
         for c, (fw, fh, erode, sig) in enumerate(INGEST):
             wi, hi = int(W * fw), int(H * fh)
             d, col = orc.ingest_frame(depth, color, wi, hi, erode=bool(erode), depth_filter=sig > 0, sigmaD=sig if sig > 0 else 2.0)
-            assert np.array_equal(bits(d), bits(g[f"ingest{k}_{c}_depth"])) and np.array_equal(col, g[f"ingest{k}_{c}_color"]), (k, c)
+            assert matches(np.asarray(d, F), g, f"ingest{k}_{c}_depth") and matches(col, g, f"ingest{k}_{c}_color"), (k, c)       # bit for bit (stored as CRC32)
 
 
 def close_ulps(a, b):

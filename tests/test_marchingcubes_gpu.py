@@ -9,7 +9,7 @@ import pytest
 
 from bundlefusion_b200 import _capi as capi
 from bundlefusion_b200 import synth
-from bundlefusion_b200.marching_cubes import CUDAMarchingCubesHashSDF, marching_cubes_params
+from bundlefusion_b200.marching_cubes import CUDAMarchingCubesHashSDF, marching_cubes_params, merge_close_vertices, remove_duplicate_faces
 from bundlefusion_b200.scene_rep import CUDASceneRepHashSDF, camera_params, default_hash_params
 from oracle import oracle as orc
 from tests.test_marchingcubes_reference_emulated import canon
@@ -58,15 +58,25 @@ def test_marching_cubes_matches_oracle_bit_for_bit(cuda_device, tmp_path):
     assert mc.extractIsoSurface(gpu, box[0], box[1], True) == 3 * (len(want) + len(wantb))
     got2, _ = soup_triangles(mc)
     assert np.array_equal(canon(got2[len(want):]), canon(wantb)) and np.array_equal(got2[:len(want)], got)
-    # saveMesh: merge / de-duplicate / PLY; an existing file is kept and the name counts up; the buffer is cleared
+    # saveMesh: merge / de-duplicate / PLY; an existing file is kept and the name counts up; the buffer is cleared.  The soup's order is the
+    # order of the atomic appends, so it differs between extractions, and with it which vertex of a merged cluster survives: each file is
+    # checked against the soup it was made from.
     mc.clearMeshBuffer()
     mc.extractIsoSurface(gpu)
+    soup1 = mc.soup()
     path = str(tmp_path / "scans" / "scan.ply")
     first = mc.saveMesh(path)
     assert first == path and os.path.exists(path) and mc.soup()[0].shape[0] == 0
     mc.extractIsoSurface(gpu)
+    soup2 = mc.soup()
+    assert np.array_equal(canon(soup_triangles(mc)[0]), canon(want))
     second = mc.saveMesh(path, transform=np.diag([2.0, 2.0, 2.0, 1.0]).astype(np.float32))
     assert second == str(tmp_path / "scans" / "scan1.ply") and os.path.exists(second)
+
+    def merged(soup):
+        pos, col = soup
+        p, c, f = merge_close_vertices(pos, col, np.arange(len(pos), dtype=np.uint32).reshape(-1, 3), 0.00001)
+        return p, (c * 255).astype(np.uint8), remove_duplicate_faces(f)
 
     def read_ply(f):
         head, body = open(f, "rb").read().split(b"end_header\n", 1)
@@ -80,7 +90,10 @@ def test_marching_cubes_matches_oracle_bit_for_bit(cuda_device, tmp_path):
     v2, f2 = read_ply(second)
     # the merged mesh: every cell edge vertex once instead of once per adjoining triangle; (almost) every triangle survives
     assert len(v1) < len(want) and 0.98 * len(want) < len(f1) <= len(want) and f1["i"].max() <= len(v1) - 1 and f1["i"].min() == 0
-    assert len(v2) == len(v1) and np.allclose(v2["p"], 2.0 * v1["p"], rtol=1e-6, atol=0) and np.array_equal(v2["c"], v1["c"])
+    for (v, fa), soup, scale in (((v1, f1), soup1, 1.0), ((v2, f2), soup2, 2.0)):
+        p, c, f = merged(soup)
+        assert len(v) == len(p) and np.allclose(v["p"], scale * p, rtol=1e-6, atol=0) and np.array_equal(v["c"], c) and np.array_equal(fa["i"], f.astype(np.int32))
+    assert abs(len(v2) - len(v1)) <= 1e-3 * len(v1) and abs(len(f2) - len(f1)) <= 1e-3 * len(f1)
     mc.close(); gpu.close()
 
 

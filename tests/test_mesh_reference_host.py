@@ -11,6 +11,7 @@ import pytest
 
 from bundlefusion_b200 import marching_cubes as mc
 from oracle import oracle as orc
+from tests._golden import input_crc, load
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 GOLDEN = os.path.join(HERE, "golden", "mesh_reference_host.npz")
@@ -73,17 +74,33 @@ def test_mesh_cleanup_and_ply_equal_the_references_golden(tmp_path, name, transf
     assert open(path, "rb").read() == g["ply_" + key].tobytes()                            # the file the reference writes, byte for byte
 
 
-@pytest.mark.skipif(not os.path.exists(REF_SO), reason="oracle/_ref/libref_mesh_host.so not built (needs /root/reference: python oracle/build_ref.py)")
-def test_live_against_the_references_mesh_classes(tmp_path):
-    g = np.load(GOLDEN)
+def live_soups():
+    """four more soups: other visiting orders (which vertex of a cluster survives depends on it), jitter, mirrored through the origin, a transform"""
     rng = np.random.default_rng(11)
+    out = []
     for it in range(4):
-        tri = soups()["a"][rng.permutation(1200)[:400]].copy()                            # another visiting order: which vertex of a cluster survives depends on it
+        tri = soups()["a"][rng.permutation(1200)[:400]].copy()
         tri[..., :3] += rng.uniform(-1.2e-5, 1.2e-5, tri[..., :3].shape).astype(np.float32) * (it % 2)
-        tri[..., :3] *= np.float32(1 - 2 * (it // 2))                                      # mirrored through the origin
-        lp, rp = str(tmp_path / "l.ply"), str(tmp_path / "r.ply")
-        p, c, f = library_save(tri, TRANSFORM if it == 3 else None, lp)
-        wp, wc, wf = reference_save(tri, TRANSFORM if it == 3 else None, rp)
+        tri[..., :3] *= np.float32(1 - 2 * (it // 2))
+        out.append((tri, TRANSFORM if it == 3 else None))
+    return out
+
+
+def test_live_against_the_references_mesh_classes(tmp_path):
+    """the reference's results on live_soups() -- merged vertices, colours, faces, PLY bytes -- are stored in tests/golden/reference_host_cases.npz
+    (scripts/make_golden_reference_host_cases.py); where oracle/_ref is built, its classes compute them again"""
+    g, h = np.load(GOLDEN), load("reference_host_cases.npz")
+    live = os.path.exists(REF_SO)
+    for it, (tri, transform) in enumerate(live_soups()):
+        assert int(h[f"mesh{it}_input_crc"]) == input_crc(tri), it
+        wp, wc, wf, wply = (h[f"mesh{it}_{k}"] for k in ("pos", "col", "faces", "ply"))
+        lp = str(tmp_path / "l.ply")
+        p, c, f = library_save(tri, transform, lp)
         assert np.array_equal(p.view(np.uint32), wp.view(np.uint32)) and np.array_equal(c, wc) and np.array_equal(f, wf)
-        assert open(lp, "rb").read() == open(rp, "rb").read()
-    assert np.array_equal(reference_save(soups()["b"], None, str(tmp_path / "g.ply"))[2], g["faces_b"])       # the golden file is what the reference produces now
+        assert open(lp, "rb").read() == wply.tobytes()
+        if live:
+            rp = str(tmp_path / "r.ply")
+            rp_, rc_, rf_ = reference_save(tri, transform, rp)
+            assert np.array_equal(rp_.view(np.uint32), wp.view(np.uint32)) and np.array_equal(rc_, wc) and np.array_equal(rf_, wf) and open(rp, "rb").read() == wply.tobytes()
+    if live:
+        assert np.array_equal(reference_save(soups()["b"], None, str(tmp_path / "g.ply"))[2], g["faces_b"])       # the golden file is what the reference produces now

@@ -3,8 +3,10 @@
 tests/golden/sens_reference_sensordata.npz (raw colour with raw and with stb-zlib depth -- JPEG / PNG can only be written through the reference's Windows-only uplink codec).
   * the library's reader on the reference's files: every header field and every frame;
   * the library's writer: with raw depth the FILE is the reference's, byte for byte; with zlib depth (another deflate encoder) the reference's loadFromFile + decompress
-    give back the frames (live, where oracle/_ref is built);
-  * a file with JPEG colour is read by both readers into the same pixels (live)."""
+    give back the frames;
+  * a file with JPEG colour is read by both readers into the same pixels.
+What the reference's reader made of the last two files is stored in tests/golden/reference_host_cases.npz (scripts/make_golden_reference_host_cases.py), with
+the files; where oracle/_ref is built, the reference reads them again."""
 import ctypes as C
 import io
 import os
@@ -14,6 +16,7 @@ import numpy as np
 import pytest
 
 from bundlefusion_b200 import sens, synth
+from tests._golden import load
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 GOLDEN = os.path.join(HERE, "golden", "sens_reference_sensordata.npz")
@@ -45,6 +48,8 @@ class RefSensorData:
         arrs = [np.ascontiguousarray(a) for a in (K, rgb, depth, poses, ts)]
         assert self.L.ref_sensordata_write(path.encode(), w, h, arrs[0].ctypes.data, 1000.0, depth_type, NAME.encode(), n, arrs[1].ctypes.data, arrs[2].ctypes.data, arrs[3].ctypes.data,
                                            arrs[4].ctypes.data) == 0
+
+    READ = ("dims", "calib", "shift", "name", "rgb", "depth", "poses", "ts")
 
     def read(self, path, w, h, cap):
         dims = np.zeros(8, np.uint32); calib = np.zeros((4, 4, 4), np.float32); shift = C.c_float(0); name = C.create_string_buffer(256)
@@ -85,30 +90,45 @@ def test_reader_on_the_references_files_and_writer_byte_for_byte(tmp_path, zl):
         assert open(q, "rb").read() == g["file_depth0"].tobytes()
 
 
-@pytest.mark.skipif(not os.path.exists(REF_SO), reason="oracle/_ref/libref_sensordata_host.so not built (needs /root/reference: python oracle/build_ref.py)")
-def test_live_against_the_references_sensor_data_class(tmp_path):
+def jpeg_blobs(rgb):
+    """the colour of sequence() encoded by libjpeg (through Pillow); the tests read the blobs stored in reference_host_cases.npz, the encoder's output being version dependent"""
     from PIL import Image
-    R = RefSensorData()
-    g = np.load(GOLDEN)
-    K, rgb, depth, poses, ts = sequence()
-    for zl in (0, 1):                                                    # the golden files are what the reference writes now
-        p = str(tmp_path / f"r{zl}.sens")
-        R.write(p, K, rgb, depth, poses, ts, zl)
-        assert open(p, "rb").read() == g[f"file_depth{zl}"].tobytes()
-    # the library's zlib-depth file through the reference's loadFromFile / decompress*
-    q = str(tmp_path / "libz.sens")
-    library_write(q, K, rgb, depth, poses, ts, True)
-    dims, calib, shift, name, rrgb, rdepth, rposes, rts = R.read(q, W, H, N)
-    assert list(dims) == [W, H, W, H, 0, 1, N, 0] and shift == 1000.0 and name == NAME and np.array_equal(calib[0], K) and np.array_equal(calib[3], np.eye(4))
-    assert np.array_equal(rrgb, rgb) and np.array_equal(rdepth, depth) and np.array_equal(rposes.view(np.uint32), poses.view(np.uint32)) and np.array_equal(rts, ts)
-    # JPEG colour (a file laid out as saveToFile lays it out, the colour encoded by libjpeg): both readers decode the same pixels
-    from tests.test_sens_reference_stb import assemble_sens
     blobs = []
     for i in range(N):
         bio = io.BytesIO(); Image.fromarray(rgb[i]).save(bio, "JPEG", quality=85 + 5 * i, subsampling=i % 3); blobs.append(bio.getvalue())
-    j = str(tmp_path / "jpeg.sens")
+    return blobs
+
+
+def write_library_and_jpeg_files(d, blobs):
+    """the two files the reference's reader is given: the library's zlib-depth file and a file with JPEG colour laid out as saveToFile lays it out"""
+    from tests.test_sens_reference_stb import assemble_sens
+    K, rgb, depth, poses, ts = sequence()
+    q, j = os.path.join(d, "libz.sens"), os.path.join(d, "jpeg.sens")
+    library_write(q, K, rgb, depth, poses, ts, True)
     assemble_sens(j, W, H, blobs, [depth[i].tobytes() for i in range(N)], sens.COLOR_JPEG, sens.DEPTH_RAW_USHORT)
-    dims, _, _, _, rrgb, rdepth, _, _ = R.read(j, W, H, N)
+    return q, j
+
+
+def test_live_against_the_references_sensor_data_class(tmp_path):
+    g, h = np.load(GOLDEN), load("reference_host_cases.npz")
+    K, rgb, depth, poses, ts = sequence()
+    q, j = write_library_and_jpeg_files(str(tmp_path), [h[f"sd_jpeg{i}"].tobytes() for i in range(N)])
+    assert open(q, "rb").read() == h["sd_libz_file"].tobytes(), "the library writes another file than the reference read"
+    stored = {f: tuple(h[f"sd_{f}_{k}"] for k in RefSensorData.READ) for f in ("libz", "jpeg")}
+    if os.path.exists(REF_SO):
+        R = RefSensorData()
+        for zl in (0, 1):                                                # the golden files are what the reference writes now
+            p = str(tmp_path / f"r{zl}.sens")
+            R.write(p, K, rgb, depth, poses, ts, zl)
+            assert open(p, "rb").read() == g[f"file_depth{zl}"].tobytes()
+        for f, path in (("libz", q), ("jpeg", j)):                       # the stored reads are what the reference's reader returns now
+            assert all(np.array_equal(a, b) for a, b in zip(R.read(path, W, H, N), stored[f]))
+    # the library's zlib-depth file through the reference's loadFromFile / decompress*
+    dims, calib, shift, name, rrgb, rdepth, rposes, rts = stored["libz"]
+    assert list(dims) == [W, H, W, H, 0, 1, N, 0] and shift == 1000.0 and str(name) == NAME and np.array_equal(calib[0], K) and np.array_equal(calib[3], np.eye(4))
+    assert np.array_equal(rrgb, rgb) and np.array_equal(rdepth, depth) and np.array_equal(rposes.view(np.uint32), poses.view(np.uint32)) and np.array_equal(rts, ts)
+    # JPEG colour: both readers decode the same pixels
+    dims, _, _, _, rrgb, rdepth, _, _ = stored["jpeg"]
     r = sens.SensorDataReader(j)
     assert list(dims[:7]) == [W, H, W, H, 2, 0, N]
     for i in range(N):

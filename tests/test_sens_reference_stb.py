@@ -10,11 +10,12 @@ import ctypes as C
 import io
 import os
 import struct
+import zlib
 
 import numpy as np
-import pytest
 
 from bundlefusion_b200 import sens
+from tests._golden import load, matches
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 GOLDEN = os.path.join(HERE, "golden", "sens_reference_stb.npz")
@@ -141,7 +142,7 @@ def test_jpeg_and_png_decoders_bit_exact_with_the_references_stb_golden():
     assert n >= 80 and sum(1 for i in range(n) if b"\xff\xc2" in g[f"jpeg_{i}"].tobytes()) >= 20
     for i in range(n):
         got = sens.decode_jpeg(g[f"jpeg_{i}"].tobytes())
-        assert got.shape == g[f"jpeg_rgb_{i}"].shape and np.array_equal(got, g[f"jpeg_rgb_{i}"]), i
+        assert matches(got, g, f"jpeg_rgb_{i}"), i
     for i in range(int(g["num_png"])):
         assert np.array_equal(sens.decode_png(g[f"png_{i}"].tobytes()), g[f"png_rgb_{i}"]), i
 
@@ -158,35 +159,56 @@ def test_reader_on_a_file_with_the_references_payloads(tmp_path):
     assert len(r) == len(ids)
     for k, i in enumerate(ids):
         du, cu = r.frame_raw(k)
-        assert np.array_equal(du, depth) and np.array_equal(cu, g[f"jpeg_rgb_{i}"])
+        assert np.array_equal(du, depth) and matches(cu, g, f"jpeg_rgb_{i}")
         d, c, _, _ = r.frame(k)
-        assert np.array_equal(c[..., :3], g[f"jpeg_rgb_{i}"]) and np.array_equal(np.isfinite(d), depth > 0)
+        assert matches(c[..., :3], g, f"jpeg_rgb_{i}") and np.array_equal(np.isfinite(d), depth > 0)
     r.close()
 
 
-@pytest.mark.skipif(not os.path.exists(REF_SO), reason="oracle/_ref/libref_sens_host.so not built (needs /root/reference: python oracle/build_ref.py)")
-def test_live_against_the_references_stb(tmp_path):
-    """where the reference's codecs are built: the golden file is what they produce now, more random streams decode identically, and depth written by this library's
-    writer (system zlib) is read back by the reference's inflate"""
-    R = RefStb()
-    g = np.load(GOLDEN)
-    jpegs, pngs, depth = make_streams()
-    for i in (0, 7, len(jpegs) - 1):
-        assert np.array_equal(R.decode(g[f"jpeg_{i}"].tobytes()), g[f"jpeg_rgb_{i}"])
+def more_jpegs():
+    """60 more random streams (Pillow's libjpeg: sizes, qualities, subsampling, restart markers, progressive); the tests read the streams stored in
+    reference_host_cases.npz, the encoder's output being version dependent"""
     from PIL import Image
     rng = np.random.default_rng(77)
+    out = []
     for _ in range(60):
         h, w = int(rng.integers(1, 90)), int(rng.integers(1, 90))
         img = picture(rng, h, w)
         bio = io.BytesIO()
         Image.fromarray(img).save(bio, "JPEG", quality=int(rng.integers(5, 101)), subsampling=int(rng.integers(0, 3)), restart_marker_blocks=int(rng.integers(0, 4)),
                                   progressive=bool(rng.integers(0, 2)))
-        assert np.array_equal(sens.decode_jpeg(bio.getvalue()), R.decode(bio.getvalue())), (h, w)
+        out.append(bio.getvalue())
+    return out
+
+
+def library_zlib_depth(path, depth):
+    """the depth payload of a file this library's writer (system zlib) makes"""
     K = np.eye(4, dtype=np.float32)
-    p = str(tmp_path / "w.sens")
-    wr = sens.SensorDataWriter(p, 160, 120, K, depth_shift=1000.0, zlib_depth=True)
+    wr = sens.SensorDataWriter(path, 160, 120, K, depth_shift=1000.0, zlib_depth=True)
     wr.append(depth, np.zeros((120, 160, 3), np.uint8), K)
     wr.finish()
     from tests.test_sens_io import python_reader
-    _, fr = python_reader(p)
-    assert R.zlib_decode(fr[0][4], depth.nbytes) == depth.tobytes()
+    _, fr = python_reader(path)
+    return fr[0][4]
+
+
+def test_live_against_the_references_stb(tmp_path):
+    """more random streams decode as the reference's stb_image decodes them, and depth written by this library's writer is read back by the reference's
+    inflate.  The reference's results are stored in tests/golden/reference_host_cases.npz (scripts/make_golden_reference_host_cases.py); where its codecs
+    are built, they compute them again, and the golden file above is checked to be what they produce now."""
+    g, h = np.load(GOLDEN), load("reference_host_cases.npz")
+    jpegs, pngs, depth = make_streams()
+    more = [h[f"stb_jpeg{i}"].tobytes() for i in range(int(h["stb_num_jpeg"]))]
+    assert len(more) == 60
+    for i, b in enumerate(more):
+        assert matches(sens.decode_jpeg(b), h, f"stb_jpeg_rgb{i}"), i
+    z = library_zlib_depth(str(tmp_path / "w.sens"), depth)
+    assert z == h["stb_lib_zlib"].tobytes(), "the library writes another payload than the reference read"
+    assert int(h["stb_lib_zlib_decoded_crc"]) == zlib.crc32(depth.tobytes())        # the reference's inflate gave back the depth
+    if os.path.exists(REF_SO):
+        R = RefStb()
+        for i in (0, 7, len(jpegs) - 1):
+            assert matches(R.decode(g[f"jpeg_{i}"].tobytes()), g, f"jpeg_rgb_{i}")
+        for i, b in enumerate(more):
+            assert matches(R.decode(b), h, f"stb_jpeg_rgb{i}"), i
+        assert R.zlib_decode(z, depth.nbytes) == depth.tobytes()

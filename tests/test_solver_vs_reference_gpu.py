@@ -1,6 +1,7 @@
-"""Parity of the bundle-adjustment solver against the REFERENCE'S OWN CUDA solver (oracle/_ref/libref_solver*.so:
-FL/Solver/SolverBundling.cu + FL/SBA.cu built for sm_100a with the compatibility patch of oracle/build_ref.py), on identical
-correspondences, cache frames and initial poses, on the GPU.  This is what pins the CPU oracle (oracle/solver_oracle.c) too: the
+"""Parity of the bundle-adjustment solver against the REFERENCE'S OWN CUDA solver (FL/Solver/SolverBundling.cu + FL/SBA.cu built for sm_100a
+with the compatibility patch of oracle/build_ref.py), on identical correspondences, cache frames and initial poses, on the GPU.  The reference's
+results are stored in tests/golden/solver_vs_reference_cuda.npz (scripts/make_golden_reference_cuda.py ran its kernels on a B200, IEEE and
+--use_fast_math builds), each with a CRC of the inputs it was computed from.  This is what pins the CPU oracle (oracle/solver_oracle.c) too: the
 same cases are run through it and compared with the reference's output.
 
 Tolerance (BASELINE.json north_star): solved poses within 1e-4 relative L2.  The reference accumulates with float atomics, so its
@@ -14,7 +15,7 @@ from bundlefusion_b200 import _capi as capi
 from bundlefusion_b200 import synth
 from bundlefusion_b200.solver import CUDASolverBundling, DeviceCache
 from oracle import oracle as orc
-from oracle import ref_solver
+from tests._golden import input_crc, load
 
 pytestmark = pytest.mark.gpu
 TOL = 1e-4
@@ -45,19 +46,11 @@ def run_ours(dev, prob, corr, n_gn, n_pcg, wS, wD=None, wC=None, cache=None):
     return np.c_[rot.cpu().numpy(), trans.cpu().numpy()], s.getStats()
 
 
-def run_ref(dev, prob, corr, n_gn, n_pcg, wS, wD=None, wC=None, cache=None, fast=True):
-    N = len(prob["init_rot"])
-    corr_t, rot, trans, valid = _dev_inputs(dev, prob, corr)
-    s = ref_solver.ReferenceSolverBundling(N, max(len(corr), 1000 * N), dev, fast_math=fast)
-    conv = s.solve(corr_t, len(corr), valid, N, n_gn, n_pcg, wS, wD, wC, d_rot=rot, d_trans=trans, cudaCache=cache,
-                   record_convergence=len(corr) > 0)    # EvalResidual launches a 0-block grid when there are no correspondences
-    return np.c_[rot.cpu().numpy(), trans.cpu().numpy()], conv, s
-
-
-@pytest.fixture(autouse=True)
-def _need_ref():
-    if not ref_solver.available(True) or not ref_solver.available(False):
-        pytest.skip("oracle/_ref/libref_solver*.so not built (needs /root/reference at build time)")
+def reference(key, prob):
+    """the reference's stored results of case `key`, after checking they were computed from these inputs"""
+    g = load("solver_vs_reference_cuda.npz")
+    assert int(g[key + "_input_crc"]) == input_crc(prob), f"the stored reference results of {key} were computed from other inputs"
+    return lambda name: g[f"{key}_{name}"]
 
 
 @pytest.mark.parametrize("fast", [True, False])
@@ -66,7 +59,8 @@ def test_sparse_solve_matches_reference_cuda(cuda_device, n_images, degree, n_gn
     cpp = 256 if n_images == 2 else 25
     prob = synth.make_ba_problem(n_images, degree=degree, corr_per_pair=cpp, noise=0.002, seed=5)
     w = [1.0] * n_gn
-    x_ref, conv, _ = run_ref(cuda_device, prob, prob["corr"], n_gn, n_pcg, w, fast=fast)
+    ref = reference(f"sparse_{n_images}_{int(fast)}", prob)
+    x_ref, conv = ref("x"), ref("conv")
     x_our, st = run_ours(cuda_device, prob, prob["corr"], n_gn, n_pcg, w)
     o = orc.solve_sparse(prob["corr"], prob["init_rot"], prob["init_trans"], n_gn, n_pcg)
     x_orc = np.c_[o["rot"], o["trans"]]
@@ -115,10 +109,10 @@ def test_dense_only_matches_reference_cuda(cuda_device):
     empty = prob["corr"][:0]
     sens, o = oracle_sensitivity(prob, empty, 2, 10, wS, wD, wC)
     assert sens < 1e-5 and orc.decision_margin(o["trace"]) > 0.3, "test problem is not well-posed"
-    x_ref, _, s = run_ref(cuda_device, prob, empty, 2, 10, wS, wD, wC, cache=cache, fast=False)
-    x_ref2, _, _ = run_ref(cuda_device, prob, empty, 2, 10, wS, wD, wC, cache=cache, fast=False)
+    ref = reference("dense_only", prob)
+    x_ref, x_ref2 = ref("x"), ref("x2")                                     # two runs of the reference
     x_our, st = run_ours(cuda_device, prob, empty, 2, 10, wS, wD, wC, cache=cache)
-    n_overlap_ref = int(s._bufs["d_numDenseOverlappingImages"].cpu().numpy()[0])
+    n_overlap_ref = int(ref("overlap"))
     assert st["dense_overlap_pairs"] == n_overlap_ref == o["overlap_pairs"]
     assert rel_l2(x_ref2, x_ref) < TOL, "the reference does not reproduce itself on this problem"
     assert rel_l2(x_our, x_ref) < TOL
@@ -138,11 +132,12 @@ def test_dense_only_chaotic_configuration_is_bounded_by_its_own_sensitivity(cuda
     empty = prob["corr"][:0]
     sens, o = oracle_sensitivity(prob, empty, 3, 60, wS, wD, wC, n=6)
     assert sens > 1e-3, "this configuration is expected to be chaotic (documented above)"
-    x_ref, _, _ = run_ref(cuda_device, prob, empty, 3, 60, wS, wD, wC, cache=cache, fast=False)
+    ref = reference("chaotic", prob)
+    x_ref = ref("x")
     x_our, _ = run_ours(cuda_device, prob, empty, 3, 60, wS, wD, wC, cache=cache)
     assert rel_l2(x_our, x_ref) < max(TOL, 3 * sens)
     # the first Gauss-Newton step truncated before the stagnation (10 PCG iterations) is decided identically by everyone
-    x_ref1, _, _ = run_ref(cuda_device, prob, empty, 1, 10, wS[:1], wD[:1], wC[:1], cache=cache, fast=False)
+    x_ref1 = ref("x1")
     x_our1, _ = run_ours(cuda_device, prob, empty, 1, 10, wS[:1], wD[:1], wC[:1], cache=cache)
     assert rel_l2(x_our1, x_ref1) < 2e-4
 
@@ -154,10 +149,11 @@ def test_local_chunk_sparse_plus_dense_matches_reference_cuda(cuda_device, wC, f
     prob = synth.make_dense_ba_problem(11, stride=3, W=320, H=240)
     cache = DeviceCache(prob["caches"], prob["intrinsics"], cuda_device)
     wS, wD = [1.0, 1.0], [1.0, 2.0]
-    x_ref, _, s = run_ref(cuda_device, prob, prob["corr"], 2, 100, wS, wD, wC, cache=cache, fast=fast)
+    ref = reference("local", prob)
+    x_ref = ref(f"{int(wC[0] > 0)}_{int(fast)}_x")
     x_our, st = run_ours(cuda_device, prob, prob["corr"], 2, 100, wS, wD, wC, cache=cache)
     o = orc.solve(prob["corr"], prob["init_rot"], prob["init_trans"], 2, 100, wS, wD, wC, prob["caches"], prob["intrinsics"])
-    assert st["dense_overlap_pairs"] == int(s._bufs["d_numDenseOverlappingImages"].cpu().numpy()[0])
+    assert st["dense_overlap_pairs"] == int(ref(f"{int(wC[0] > 0)}_{int(fast)}_overlap"))
     assert rel_l2(x_our, x_ref) < TOL
     assert rel_l2(np.c_[o["rot"], o["trans"]], x_ref) < TOL
 
@@ -171,10 +167,11 @@ def test_dense_system_matches_reference_cuda(cuda_device):
     cache = DeviceCache(prob["caches"], prob["intrinsics"], cuda_device)
     N = 6
     # one GN iteration with zero PCG iterations leaves the poses untouched and the system of iteration 0 in the buffers
-    x_ref, _, s = run_ref(cuda_device, prob, prob["corr"][:0], 1, 0, [0.0], [1.0], [0.1], cache=cache, fast=False)
+    ref = reference("dense_system", prob)
+    x_ref = ref("x")
     np.testing.assert_array_equal(x_ref, np.c_[prob["init_rot"], prob["init_trans"]])
-    JtJ_ref = s._bufs["d_denseJtJ"].cpu().numpy().reshape(6 * N, 6 * N)
-    Jtr_ref = s._bufs["d_denseJtr"].cpu().numpy()
+    JtJ_ref = ref("JtJ")
+    Jtr_ref = ref("Jtr")
     JtJ, Jtr, _ = orc.build_dense(prob["init_rot"], prob["init_trans"], prob["caches"], prob["intrinsics"], 1.0, 0.1)
     assert np.linalg.norm(JtJ_ref) > 0
     assert rel_l2(JtJ, JtJ_ref) < TOL
@@ -203,8 +200,8 @@ def test_dense_term_beyond_64_images_matches_reference_cuda(cuda_device):
     N = 72
     prob = synth.make_dense_ba_problem(N, stride=1, start=60, corr_per_pair=8, W=320, H=240)
     cache = DeviceCache(prob["caches"], prob["intrinsics"], cuda_device)
-    x_ref, _, s = run_ref(cuda_device, prob, prob["corr"][:0], 1, 0, [0.0], [1.0], [0.1], cache=cache, fast=False)
-    JtJ_ref = s._bufs["d_denseJtJ"].cpu().numpy().reshape(6 * N, 6 * N); Jtr_ref = s._bufs["d_denseJtr"].cpu().numpy()
+    ref = reference("beyond64", prob)
+    JtJ_ref = np.zeros((6 * N, 6 * N), np.float32); JtJ_ref[6:, 6:] = ref("JtJ"); Jtr_ref = ref("Jtr")      # stored without the fixed variable 0's rows / columns
     corr_t, rot, trans, valid = _dev_inputs(cuda_device, prob, prob["corr"][:0])
     sv = CUDASolverBundling(N, 1000 * N, cuda_device)
     sv.solve(corr_t, 0, valid, N, 1, 0, [0.0], [1.0], [0.1], d_rotationAnglesUnknowns=rot, d_translationUnknowns=trans, cudaCache=cache)
@@ -216,9 +213,9 @@ def test_dense_term_beyond_64_images_matches_reference_cuda(cuda_device):
     assert rel_l2(JtJ_our[6:, 6:], JtJ_ref[6:, 6:]) < TOL and rel_l2(Jtr_our[6:], Jtr_ref[6:]) < TOL
     assert np.array_equal(JtJ_our[6:, 6:] != 0, JtJ_ref[6:, 6:] != 0), "same block sparsity as the reference's dense matrix"
     wS, wD, wC = [1.0, 1.0], [1.0, 2.0], [0.1, 0.1]
-    x_ref, _, s = run_ref(cuda_device, prob, prob["corr"], 2, 15, wS, wD, wC, cache=cache, fast=False)
+    x_ref = ref("x")
     x_our, st = run_ours(cuda_device, prob, prob["corr"], 2, 15, wS, wD, wC, cache=cache)
-    assert st["dense_overlap_pairs"] == int(s._bufs["d_numDenseOverlappingImages"].cpu().numpy()[0])
+    assert st["dense_overlap_pairs"] == int(ref("overlap"))
     assert rel_l2(x_our, x_ref) < TOL
 
 
@@ -227,8 +224,9 @@ def test_max_residual_and_pose_stubs_match_reference_cuda(cuda_device):
     dev = cuda_device
     prob = synth.make_ba_problem(8, degree=7, corr_per_pair=25, noise=0.0, perturb_rot=0.0, perturb_trans=0.0)
     prob["corr"]["pj"][333] += np.array([0.0, 0.4, 0.0], np.float32)
-    x_ref, _, s = run_ref(dev, prob, prob["corr"], 1, 1, [1.0], fast=False)
-    v_ref, i_ref = s.max_residual()
+    ref = reference("maxres", prob)
+    x_ref = ref("x")
+    v_ref, i_ref = float(ref("v")), int(ref("i"))
     v_orc, i_orc = orc.max_residual(prob["corr"], x_ref[:, :3].astype(np.float32).copy(), x_ref[:, 3:].astype(np.float32).copy())
     assert i_ref == i_orc and abs(v_ref - v_orc) < 1e-5
     # pose <-> matrix stubs, ours against the reference's, on poses with small, moderate and near-pi rotations
@@ -236,19 +234,17 @@ def test_max_residual_and_pose_stubs_match_reference_cuda(cuda_device):
     N = 64
     rot = (rng.standard_normal((N, 3)) * np.r_[np.full(16, 1e-4), np.full(32, 0.5), np.full(16, 1.6)][:, None]).astype(np.float32)
     trans = rng.standard_normal((N, 3)).astype(np.float32)
-    outs = []
-    L_our = capi.lib()
-    L_our.bfSetStream(None)
-    for L in (s.L, L_our):
-        r = torch.from_numpy(rot).to(dev); t = torch.from_numpy(trans).to(dev)
-        T = torch.zeros(N * 16, device=dev); Ti = torch.zeros(N * 16, device=dev); T2 = torch.zeros(N * 16, device=dev)
-        r2 = torch.zeros_like(r); t2 = torch.zeros_like(t); valid = torch.ones(N, dtype=torch.int32, device=dev)
-        torch.cuda.synchronize()
-        P = C.c_void_p
-        L.convertLiePosesToMatricesCU(P(r.data_ptr()), P(t.data_ptr()), C.c_uint(N), P(T.data_ptr()), P(Ti.data_ptr()))
-        L.convertMatricesToPosesCU(P(T.data_ptr()), C.c_uint(N), P(r2.data_ptr()), P(t2.data_ptr()), P(valid.data_ptr()))
-        L.convertPosesToMatricesCU(P(r2.data_ptr()), P(t2.data_ptr()), C.c_uint(N), P(T2.data_ptr()), P(valid.data_ptr()))
-        torch.cuda.synchronize()
-        outs.append([x.cpu().numpy() for x in (T, Ti, r2, t2, T2)])
-    for a, b, tol in zip(outs[0], outs[1], (2e-6, 1e-5, 2e-4, 2e-4, 2e-4)):
-        np.testing.assert_allclose(b, a, atol=tol)
+    L = capi.lib()
+    L.bfSetStream(None)
+    r = torch.from_numpy(rot).to(dev); t = torch.from_numpy(trans).to(dev)
+    T = torch.zeros(N * 16, device=dev); Ti = torch.zeros(N * 16, device=dev); T2 = torch.zeros(N * 16, device=dev)
+    r2 = torch.zeros_like(r); t2 = torch.zeros_like(t); valid = torch.ones(N, dtype=torch.int32, device=dev)
+    torch.cuda.synchronize()
+    P = C.c_void_p
+    L.convertLiePosesToMatricesCU(P(r.data_ptr()), P(t.data_ptr()), C.c_uint(N), P(T.data_ptr()), P(Ti.data_ptr()))
+    L.convertMatricesToPosesCU(P(T.data_ptr()), C.c_uint(N), P(r2.data_ptr()), P(t2.data_ptr()), P(valid.data_ptr()))
+    L.convertPosesToMatricesCU(P(r2.data_ptr()), P(t2.data_ptr()), C.c_uint(N), P(T2.data_ptr()), P(valid.data_ptr()))
+    torch.cuda.synchronize()
+    stubs = reference("stubs", (rot, trans))
+    for name, x, tol in zip(("T", "Ti", "r2", "t2", "T2"), (T, Ti, r2, t2, T2), (2e-6, 1e-5, 2e-4, 2e-4, 2e-4)):
+        np.testing.assert_allclose(x.cpu().numpy(), stubs(name), atol=tol)

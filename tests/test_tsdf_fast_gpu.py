@@ -15,8 +15,8 @@ from bundlefusion_b200 import _capi as capi
 from bundlefusion_b200 import synth
 from bundlefusion_b200.scene_rep import CUDASceneRepHashSDF, camera_params, default_hash_params
 from oracle import oracle as orc
-from oracle import ref_tsdf
-from tests.test_tsdf_vs_reference_gpu import compare_states
+from tests._golden import block_crcs
+from tests.test_tsdf_vs_reference_gpu import compare_states, compare_with_reference, reference_stream
 
 pytestmark = pytest.mark.gpu
 F = np.float32
@@ -91,31 +91,40 @@ def test_fast_fused_reintegration_matches_oracle_and_exact_kernels(cuda_device):
 
 @pytest.mark.parametrize("fast_math", [False, True])
 def test_fast_stream_matches_reference_cuda(cuda_device, fast_math):
-    """the same statement against the reference's own CUDA kernels (oracle/_ref), IEEE build and --use_fast_math build"""
+    """the same statement against the reference's own CUDA kernels, IEEE build and --use_fast_math build, through their stored states
+    (tests/test_tsdf_vs_reference_gpu.py): the IEEE build's state is the oracle's -- every block's CRC equals the stored one -- and is compared
+    whole; the fast-math build's on its stored sample of blocks"""
     import torch
-    if not ref_tsdf.available(fast_math):
-        pytest.skip("oracle/_ref not built (needs /root/reference at build time)")
     W, H = 320, 240
     cam = camera_params(W, H)
     hp = default_hash_params(num_buckets=100003, num_sdf_blocks=60000)
     ours = CUDASceneRepHashSDF(hp, cuda_device, arithmetic="fast")
-    ref = ref_tsdf.ReferenceSceneRepHashSDF(hp, cuda_device, fast_math=fast_math)
     frames, dl, cl = _frames(torch, cuda_device, 6, W, H)
+    g = reference_stream(fast_math, frames)
+    cpu = None if fast_math else orc.OracleSceneRepHashSDF(hp)
     tol = 1e-4 if fast_math else SDF_TOL          # the reference's fast-math build is itself ~1e-5 away from IEEE
+
+    def compare(stage, sdf_tol):
+        if fast_math:
+            return compare_with_reference(ours.download(), g, stage, sdf_tol, exact=False)
+        rb, rv = orc.canonical_blocks(cpu.download())
+        np.testing.assert_array_equal(rb, g[f"blocks{stage}"]); np.testing.assert_array_equal(block_crcs(rv), g[f"crcs{stage}"])
+        return compare_states(ours.download(), (rb, rv), sdf_tol)
+
     for (d, c, T), dd, dc in zip(frames, dl, cl):
         ours.integrate(T, dd, dc, cam)
-        ref.integrate(T, dd, dc, cam)
-    s1 = compare_states(ours.download(), ref.download(), tol)
-    assert ours.getNumOccupiedBlocks() == ref.hp.m_numOccupiedBlocks and ours.getHeapFreeCount() == ref.getHeapFreeCount()
+        if cpu is not None: cpu.integrate(T, d, c, cam)
+    s1 = compare(1, tol)
+    assert ours.getNumOccupiedBlocks() == int(g["occupied1"]) and ours.getHeapFreeCount() == int(g["heap_free1"])
     for k in (1, 4):
         d, c, T = frames[k]
         T2 = T.copy(); T2[:3, 3] += np.array([0.011, -0.006, 0.004], F)
         ours.runOps([(capi.BF_TSDF_OP_DEINTEGRATE, k, T), (capi.BF_TSDF_OP_INTEGRATE, k, T2)], dl, cl, cam)       # fused pass
-        ref.deIntegrate(T, dl[k], cl[k], cam); ref.integrate(T2, dl[k], cl[k], cam)
-    ours.deIntegrate(frames[0][2], dl[0], cl[0], cam); ref.deIntegrate(frames[0][2], dl[0], cl[0], cam)
-    ours.garbageCollect(); ref.garbageCollect()
-    s2 = compare_states(ours.download(), ref.download(), 10 * tol)
-    assert ours.getHeapFreeCount() == ref.getHeapFreeCount()
+        if cpu is not None: cpu.deIntegrate(T, d, c, cam); cpu.integrate(T2, d, c, cam)
+    ours.deIntegrate(frames[0][2], dl[0], cl[0], cam); ours.garbageCollect()
+    if cpu is not None: cpu.deIntegrate(frames[0][2], frames[0][0], frames[0][1], cam); cpu.garbageCollect()
+    s2 = compare(2, 10 * tol)
+    assert ours.getHeapFreeCount() == int(g["heap_free2"])
     print("fast vs reference CUDA (fast_math=%s):" % fast_math, s1, s2)
 
 
